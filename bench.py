@@ -48,7 +48,14 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 3-5 block")
     ap.add_argument("--quick-configs", action="store_true", help="configs block at 20%% of the stated sizes")
     ap.add_argument("--r-default-probe", action="store_true", help=argparse.SUPPRESS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; a fixed, seeded "
+                         "sample of the genes of large outputs), so two builds can be compared output for output; "
+                         "with more than one GPU: rank 0's own shard, not the gathered results")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 # ---------------------------------------------------------------- workload
@@ -464,6 +471,32 @@ def configs_block(world, rank, dev, peak_gbs, quick=False):
     return out
 
 
+def last_step_outputs(outs, ng, m, max_genes=100000, matrix_bytes=32 << 20):
+    """What the three calls of a step return to their caller, as float64 host arrays: fitDisp MLE and MAP
+    (fitdisp_mle_*, fitdisp_map_*: the nine per-gene list members) and fitBeta (fitbeta_*: beta_mat and beta_var_mat
+    as n x p, the per-gene vectors, hat_diagonals and mu as n x m).  Rows past ng only pad a shard.  A fixed, seeded
+    sample of the genes is kept where there are more than max_genes, and of the n x m matrices as many rows as fit
+    matrix_bytes; the row indices are stored as rows_vectors and rows_matrices.  The per-gene arrays take at most
+    (23 + 2 p) * 8 * max_genes bytes (21.6 MB for the benchmark's p = 2) and the two matrices at most matrix_bytes
+    (33.6 MB), so the dump stays below 64 MB for any number of genes and samples."""
+    max_matrix_rows = min(4096, matrix_bytes // (2 * 8 * m))
+    pick = lambda k: np.sort(np.random.default_rng(0).choice(ng, k, replace=False)) if k < ng else np.arange(ng)
+    rv, rm = pick(max_genes), pick(max_matrix_rows)
+    out = {"rows_vectors": rv.astype(np.float64), "rows_matrices": rm.astype(np.float64)}
+    for prefix, d in (("fitdisp_mle_", outs[0]), ("fitdisp_map_", outs[1]), ("fitbeta_", outs[2])):
+        for k, t in d.items():
+            if t is None:
+                continue
+            v = t.detach().cpu().numpy().astype(np.float64)
+            if k in ("beta_mat", "beta_var_mat"):
+                out[prefix + k] = v.T[rv]
+            elif v.ndim == 2:
+                out[prefix + k] = v[rm, :m]
+            else:
+                out[prefix + k] = v[rv]
+    return out
+
+
 def main():
     a = parse()
     if a.r_default_probe:
@@ -609,24 +642,25 @@ def main():
         step(i, True)            # warm-up includes the event records the timed steps make
     torch.cuda.synchronize()
     launches0 = L.b200nb_kernel_launches()
-    # The timed region (exactly K steps between barrier + synchronize) is repeated REPEATS times and the MEDIAN
-    # repetition is reported (all repetitions are listed in config.timed_repeats_ms): the GPU boxes show an
+    # The K timed steps run in up to WINDOWS consecutive windows (each between barrier + synchronize) and the per-step
+    # time of the MEDIAN window is reported (all windows are listed in config.timed_windows_ms): the GPU boxes show an
     # occasional ~80 ms stall that is unrelated to the workload (it hits whatever kernel happens to be running,
-    # also with garbage collection off and zero cudaMalloc/cudaFree traffic), and a single 75 ms timed region
-    # would otherwise be at its mercy.
-    REPEATS = 3
+    # also with garbage collection off and zero cudaMalloc/cudaFree traffic), and a single timed region would
+    # otherwise be at its mercy.
+    WINDOWS = min(3, a.steps)
+    bounds = [a.steps * k // WINDOWS for k in range(WINDOWS + 1)]
     no_ev = bool(os.environ.get("B200NB_NO_STEP_EVENTS"))
-    rep_ms, rep_evs, rep_w0 = [], [], []
-    for rep in range(REPEATS):
+    win_ms, evs = [], []
+    for k in range(WINDOWS):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         t_start, t_end = ev(), ev()
         w0 = time.perf_counter()
-        if rep == 0:
+        if k == 0:
             w0_first = w0
         t_start.record()
-        evs = [step(i, not no_ev) for i in range(a.steps)]
+        evs += [step(i, not no_ev) for i in range(bounds[k], bounds[k + 1])]
         for b_ in range(NBUF if world > 1 else 0):   # the timed region ends when every gather has landed
             if pending[b_] is not None:
                 pending[b_].wait()
@@ -638,16 +672,17 @@ def main():
         tm = torch.tensor([t_start.elapsed_time(t_end)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(tm, op=dist.ReduceOp.MAX)
-        rep_ms.append(float(tm.item()))
-        rep_evs.append(evs)
+        win_ms.append(float(tm.item()))
+    # the steps that keep the clock sampler busy below rewrite `outs`: keep a device copy of the last timed step's
+    # results; the host copy and the sampling happen after the sampler has stopped
+    last_outs = [{k: t.clone() for k, t in d.items() if t is not None} for d in outs] \
+        if a.dump_outputs and rank == 0 else None
     w0 = w0_first
     w0_wall = time.time() - (time.perf_counter() - w0)
-    launches = (L.b200nb_kernel_launches() - launches0) // REPEATS
-    pick = sorted(range(REPEATS), key=lambda r_: rep_ms[r_])[REPEATS // 2]
-    total_ms = rep_ms[pick]
-    evs = rep_evs[pick]
-    cfg["timed_repeats_ms"] = [round(v, 3) for v in rep_ms]
-    cfg["timed_repeat_reported"] = "median of %d repetitions of the K-step timed region" % REPEATS
+    launches = L.b200nb_kernel_launches() - launches0
+    per_step = sorted(t / (bounds[k + 1] - bounds[k]) for k, t in enumerate(win_ms))
+    cfg["timed_windows_ms"] = [round(v, 3) for v in win_ms]
+    cfg["timed_window_reported"] = "per-step time of the median of %d windows that split the K timed steps" % WINDOWS
     # keep the GPU busy a little longer so the clock sampler sees load even for very short runs
     clocks = None
     if rank == 0:
@@ -661,13 +696,14 @@ def main():
         torch.cuda.synchronize()
         sampler.window = (w0_wall, time.time())
         clocks = sampler.stop()
+    dumped = last_step_outputs(last_outs, ng, m) if last_outs is not None else None
     if no_ev:
         evs = []
         kern_ms = {"fit_disp_mle": 1e-9, "fit_disp_map": 1e-9, "fit_beta": 1e-9}
     if os.environ.get("B200NB_BENCH_DEBUG") and rank == 0 and not no_ev:
         ct = cpu_times[max(a.warmup, 3):max(a.warmup, 3) + a.steps]
         print("cpu enqueue ms per call (max over steps):", [round(1e3 * max(c[k + 1] - c[k] for c in ct), 3) for k in range(3)],
-              "cpu total enqueue ms:", round(1e3 * (ct[-1][3] - ct[0][0]), 2), "gpu ms:", round(total_ms, 2), file=sys.stderr)
+              "cpu total enqueue ms:", round(1e3 * (ct[-1][3] - ct[0][0]), 2), "gpu ms:", round(sum(win_ms), 2), file=sys.stderr)
         print("cpu per-step [mle,map,beta] ms:", [[round(1e3 * (c[k + 1] - c[k]), 2) for k in range(3)] for c in ct], file=sys.stderr)
         print("per-step ms:", [[round(e[k].elapsed_time(e[k + 1]), 3) for k in range(3)] for e in evs], file=sys.stderr)
     for e in evs:
@@ -680,7 +716,7 @@ def main():
         total_genes = float(ngt.item())
     else:
         total_genes = float(ng)
-    ms_per_step = total_ms / a.steps
+    ms_per_step = per_step[WINDOWS // 2]
     value = total_genes / (ms_per_step * 1e-3)
 
     # ---- e2e through the C ABI with host buffers (rank-local, then max over ranks)
@@ -820,6 +856,10 @@ def main():
             "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "cpu_baseline": cpu,
             "full_pipeline": full, "genes_fitted": total_genes, "configs": cfgs}
     print(json.dumps(line))
+    if dumped is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, v in dumped.items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), v)
     if world > 1:
         dist.destroy_process_group()
 

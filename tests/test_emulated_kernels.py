@@ -43,13 +43,11 @@ def test_emulated_library_exports_the_c_abi(emu):
 import test_golden as TG          # noqa: E402
 import test_parity_gpu as TP
 import test_parity_reference_gpu as TPR      # noqa: E402
+from reference_outputs import Reference  # noqa: E402
 
-def _ref():
-    from oracle import ref as R
-    if not R.available():
-        pytest.skip("oracle/_ref not available")
-    R.build()
-    return R
+
+def _ref(case):
+    return Reference("emulated_kernels", case)
 
 
 CASES = [
@@ -88,9 +86,9 @@ CASES = [
     ("edge 7x33", lambda e, o: TP.test_edge_shapes(e, o, 7, 33)),
     ("edge 2x3000", lambda e, o: TP.test_edge_shapes(e, o, 2, 3000)),
     ("empty input", lambda e, o: TP.test_empty_input_is_a_no_op(e)),
-    ("engine vs the reference TU: fitDisp m=24", lambda e, o: TPR.test_fit_disp_vs_reference(e, o, _ref(), 300, 24, 213)),
-    ("engine vs the reference TU: fitBeta m=6", lambda e, o: TPR.test_fit_beta_vs_reference(e, _ref(), 300, 6, 222, True)),
-    ("engine vs the reference TU: general p, weights, ridge", lambda e, o: TPR.test_fit_beta_weights_ridge_general_p_vs_reference(e, _ref())),
+    ("engine vs the reference TU: fitDisp m=24", lambda e, o: TPR.test_fit_disp_vs_reference(e, o, _ref("fitDisp m=24"), 300, 24, 213)),
+    ("engine vs the reference TU: fitBeta m=6", lambda e, o: TPR.test_fit_beta_vs_reference(e, _ref("fitBeta m=6"), 300, 6, 222, True)),
+    ("engine vs the reference TU: general p, weights, ridge", lambda e, o: TPR.test_fit_beta_weights_ridge_general_p_vs_reference(e, _ref("general p"))),
     ("host input cache: content-addressed, never stale", lambda e, o: TP.test_host_cache_is_content_addressed_and_never_stale(e, o)),
     ("post-rule parity m=4 (Monte-Carlo prior variance)", lambda e, o: TP.test_post_rule_parity_every_gene(e, o, 4, 250, 0.3)),
     ("post-rule parity m=6", lambda e, o: TP.test_post_rule_parity_every_gene(e, o, 6, 300, 0.25)),

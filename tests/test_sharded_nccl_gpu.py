@@ -16,7 +16,7 @@ def test_sharded_device_pipeline_over_nccl_equals_whole():
     import torch
     n_gpu = torch.cuda.device_count()
     if n_gpu < 2:
-        pytest.skip("needs at least 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs at least 2 GPUs")
     world = 4 if n_gpu >= 4 else 2
     env = dict(os.environ)
     for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK", "MASTER_ADDR", "MASTER_PORT"):
